@@ -2,6 +2,7 @@
 """bench.py -- RenderNet forward rendering throughput on B200 (contract in the task statement).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|4|5] [--precision exact|fast] [--gather nccl|peer|none]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...      # CPU restatement of the reference's TF-1 graph, host cores
@@ -58,6 +59,25 @@ def synthetic_texture(B, rank=0):
 def bunny_voxel():
     bv = np.load(os.path.join(ROOT, "tests", "golden", "binvox.npz"))      # bit-packed copy of binvox/bunny.binvox
     return np.unpackbits(bv["bunny_bits"]).reshape(1, 64, 64, 64, 1).astype(np.float32)
+
+
+DUMP_BYTES = 64_000_000     # --dump-outputs: total size of the .npy files, headers included
+
+
+def dump_outputs(out_dir, named):
+    """Writes {name: array [N, ...]} as out_dir/<name>.npy in float32, so that two builds can be compared output for
+    output.  An array larger than its share of DUMP_BYTES is cut to a fixed, seeded sample of whole items along axis 0
+    (sorted); which items depends only on N and the share, so equal arguments select the same items."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(named) - 4096
+    for name, a in named.items():
+        a = np.asarray(a, dtype=np.float32)
+        per_item = a[0].nbytes
+        if a.nbytes > share:
+            keep = np.sort(np.random.default_rng(0).choice(a.shape[0], share // per_item, replace=False))
+            print(f"dump {name}: items {keep.tolist()} of {a.shape[0]}", file=sys.stderr)
+            a = a[keep]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -281,8 +301,9 @@ def run_ours(args, rank, world, local_rank):
         tex = synthetic_texture(B, rank) if cfg == 4 else None
         units_per_step_global = world * B
 
-    def measure(precision, with_e2e, gather_kind):
-        """-> dict(ms_step, per_rank, value, e2e..., launches) for one precision."""
+    def measure(precision, with_e2e, gather_kind, dump_dir=None):
+        """-> dict(ms_step, per_rank, value, e2e..., launches) for one precision; with dump_dir, rank 0 also writes what the
+        last timed step returned (dump_outputs)."""
         eng = build(precision, B)
         sh = ShardedRenderEngine(eng, gather_kind) if cfg != 5 else None
         if sh is not None and sh.peer is not None and not sh.verify_peer_against_nccl():
@@ -342,6 +363,19 @@ def run_ours(args, rank, world, local_rank):
                 eng.result(eng.submitted - 1)
         torch.cuda.synchronize()
         ms_total, per = timed(args.steps, False)
+        if dump_dir and rank == 0:
+            if cfg == 5:
+                if gathered is None:
+                    frames = out_frames[:len(my_poses)]
+                else:                                  # every rank's block of nchunk * B frames ends in padding
+                    bounds = [shard_bounds(nframes, world, r) for r in range(world)]
+                    frames = torch.cat([gathered[r * nchunk * B:r * nchunk * B + hi - lo] for r, (lo, hi) in enumerate(bounds)])
+                named = {"frames": frames}
+            elif cfg == 4:
+                named = dict(zip(("albedo", "normal"), sh.wait()))
+            else:
+                named = {"images": sh.wait()}
+            dump_outputs(dump_dir, {k: v.cpu().numpy() for k, v in named.items()})
         phases = None
         if args.phases and sh is not None:            # where does a step's time go: graph replay vs the gather on the compute stream
             sh.timing = []
@@ -376,8 +410,10 @@ def run_ours(args, rank, world, local_rank):
         sampler.start()
     main_prec = args.precision
     other_prec = "fast" if main_prec == "exact" else "exact"
-    M = measure(main_prec, True, args.gather)
-    clocks = sampler.stop(set(range(world))) if rank == 0 else None
+    try:
+        M = measure(main_prec, True, args.gather, args.dump_outputs)
+    finally:                                    # a failed measurement must not leave nvidia-smi sampling behind
+        clocks = sampler.stop(set(range(world))) if rank == 0 else None
     O = None if args.no_other_precision else measure(other_prec, False, "none")
 
     if rank != 0:
@@ -491,7 +527,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-precision", action="store_true")
     ap.add_argument("--no-b8", action="store_true", help="reference arm: skip the extra B=8 CPU sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline precision's outputs of the last step as DIR/<name>.npy "
+                         "(float32, at most 64 MB in all: a fixed, seeded sample of whole images when larger)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -315,6 +315,29 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert "workload" in d["config"] and d["vs_baseline"] is None
 
 
+def test_bench_dump_outputs_is_bounded_float32_and_samples_the_same_images(tmp_path):
+    """`bench.py --dump-outputs DIR`: one float32 .npy per output, whole when it fits, else the same seeded choice of whole
+    images on every run, never more than bench.DUMP_BYTES in all; the CPU reference arm refuses the option."""
+    import subprocess
+    import sys
+    import bench
+    big = np.broadcast_to(np.arange(24, dtype=np.float32)[:, None, None, None], (24, 512, 512, 3))   # 75.5 MB, image i == i
+    small = np.ones((2, 3), np.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"images": big, "small": small})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["images.npy", "small.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    imgs, s = np.load(tmp_path / "a" / "images.npy"), np.load(tmp_path / "a" / "small.npy")
+    assert imgs.dtype == np.float32 and s.dtype == np.float32 and np.array_equal(s, small)
+    picked = imgs[:, 0, 0, 0]
+    assert 10 <= len(picked) < 24 and np.all(np.diff(picked) > 0) and np.all(imgs == picked[:, None, None, None])
+    assert np.array_equal(imgs, np.load(tmp_path / "b" / "images.npy"))
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "c")],
+                       capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert p.returncode != 0 and "--dump-outputs" in p.stderr and not (tmp_path / "c").exists()
+
+
 def test_pose_matrix_vjp_matches_finite_differences_host():
     """backward.pose_matrix_jacobian_vjp: the 3 -> 12 chain rule from dL/dMinv to dL/d(azimuth, elevation, scale) (host, float64)
     against central differences of the float32 matrix construction the forward pass uses (engine.pose_to_matrix)."""
